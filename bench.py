@@ -23,13 +23,19 @@ One JSON line on stdout (rank 0):
              is the second, `first_call_value` the first (allocator cold).
   roofline   dominant kernel: algorithmic bytes / CUDA-event duration vs the
              measured HBM copy bandwidth (MEASURED_PEAKS.json)
-  cpu_baseline  the unmodified reference (baseline/_ref, kind "reference"; the
+  cpu_baseline  the unmodified reference (oracle/_ref, kind "reference"; the
              torch-CPU restatement oracle/torch_port.py, kind "port", only if the
              install is absent) timed on this box's host cores on a bounded sample
              of the same workload
 
 ``--impl reference`` times only that CPU arm (all host threads) on the same
 config and prints the same line shape with "impl": "reference".
+
+``--dump-outputs DIR`` (single GPU) writes, right after the timed steps, what they
+hand their caller as DIR/<name>.npy: ``epoch_loss`` (float64) and a fixed seeded
+sample of rows of the four trained tables with their Adagrad sums (float32, about
+34 MB at the default shape).  Ids, initial weights and the sample are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 
 import argparse
@@ -65,7 +71,12 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--exchange', default='auto', choices=['auto', 'a2a', 'dense'])
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the timed steps computed as DIR/<name>.npy (single GPU, --impl ours)')
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != 'ours' or int(os.environ.get('WORLD_SIZE', '1')) > 1):
+        ap.error('--dump-outputs is supported for --impl ours on a single GPU')
+    return a
 
 
 def workload_config(a, n_gpus):
@@ -200,13 +211,13 @@ class ClockSampler(object):
 # CPU port (cpu_baseline and the reference arm)
 # --------------------------------------------------------------------------
 
-REF_DIR = os.path.join(ROOT, 'baseline', '_ref')
+REF_DIR = os.path.join(ROOT, 'oracle', '_ref')
 
 
 def _reference_runner(a):
-    """fit_steps(lo, nsteps) on the UNMODIFIED reference (baseline/_ref, pip-installed from
-    /root/reference: `spotlight.factorization.implicit.ImplicitFactorizationModel.fit` on CPU
-    through its own public API), or None when the install is not on this box."""
+    """fit_steps(lo, nsteps) on the UNMODIFIED reference (oracle/_ref, installed by build() from a
+    reference checkout, oracle/reference.py: `spotlight.factorization.implicit.ImplicitFactorizationModel.fit`
+    on CPU through its own public API), or None when the install is not on this box."""
     if not os.path.isdir(os.path.join(REF_DIR, 'spotlight')):
         return None
     import torch
@@ -244,7 +255,7 @@ def _port_runner(a):
 def run_cpu_port(a, steps, warmup):
     """interactions/s of the reference's CPU fit() loop on this box's host cores.
 
-    kind "reference": the unmodified reference from baseline/_ref (stock code path, its own
+    kind "reference": the unmodified reference from oracle/_ref (stock code path, its own
     shuffle, sampler, autograd and the same Adagrad optimizer handed in through its
     `optimizer_func`); kind "port": oracle/torch_port.py, the same loop restated on stock
     torch CPU ops, when the install is absent.
@@ -279,7 +290,7 @@ def run_cpu_port(a, steps, warmup):
     t0 = time.perf_counter()
     fit_steps(users[lo:], items[lo:], steps)
     dt = time.perf_counter() - t0
-    what = ('unmodified reference (baseline/_ref: spotlight.factorization.implicit.'
+    what = ('unmodified reference (oracle/_ref: spotlight.factorization.implicit.'
             'ImplicitFactorizationModel.fit, use_cuda=False)' if kind == 'reference'
             else 'reference loop restated on torch CPU ops (oracle/torch_port.py)')
     return {'value': steps * B / dt, 'unit': UNIT, 'cores': best, 'kind': kind,
@@ -293,10 +304,8 @@ def main_reference(a):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    # each reference step is O(table + batch) (about a second at the default batch on the box's
-    # host cores): K and W are honoured up to a bound that keeps the arm within a few minutes
-    steps = max(1, min(a.steps, 60))
-    warm = max(1, min(a.warmup, 5))
+    # each reference step is O(table + batch): about a second at the default batch on host cores
+    steps, warm = max(1, a.steps), max(1, a.warmup)
     r = run_cpu_port(a, steps, warm)
     line = {'impl': 'reference', 'metric': METRIC, 'value': r['value'], 'unit': UNIT,
             'n_gpus': a.gpus, 'steps': steps, 'warmup': warm, 'ms_per_step': r['ms_per_step'],
@@ -329,6 +338,37 @@ def build_model(a, device_index):
     model._initialize(_Shape(a.users, a.items))
     assert model._route() == 'epoch'
     return model
+
+
+DUMP_ROWS = 32768
+DUMP_BYTES = 60 << 20       # sampled arrays; the .npy headers and epoch_loss stay well inside 64 MB
+
+
+def dump_rows(dim):
+    """Rows sampled per table: DUMP_ROWS, fewer when the two embedding tables and two bias tables,
+    each with its Adagrad sum (16 * (dim + 1) bytes a sampled row), would exceed DUMP_BYTES."""
+    return max(1, min(DUMP_ROWS, DUMP_BYTES // (16 * (dim + 1))))
+
+
+def dump_outputs(model, epoch_loss, out_dir):
+    """Write what the timed epoch hands its caller, taken right after its last step (the e2e and
+    per-kernel legs that follow keep training the same model): the epoch loss it returns and the
+    trained tables with their Adagrad sums.  A table of more than R = dump_rows(dim) rows is sampled
+    at the rows np.random.RandomState(0).choice(rows, R, replace=False), sorted."""
+    import torch
+    net, opt = model._net, model._optimizer
+    os.makedirs(out_dir, exist_ok=True)
+    out = {'epoch_loss': np.array([epoch_loss], dtype=np.float64)}
+    R = dump_rows(net.user_embeddings.weight.shape[1])
+    for name in ('user_embeddings', 'item_embeddings', 'user_biases', 'item_biases'):
+        w = getattr(net, name).weight
+        n = w.shape[0]
+        rows = np.sort(np.random.RandomState(0).choice(n, min(n, R), replace=False))
+        idx = torch.from_numpy(rows).to(w.device)
+        out[name] = w.detach().index_select(0, idx).float().cpu().numpy()
+        out[name + '_adagrad_sum'] = opt.fused_state(w).index_select(0, idx).float().cpu().numpy()
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), arr)
 
 
 def kernel_breakdown(model, users, items, a, steps):
@@ -599,6 +639,8 @@ def main_ours(a):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     value = world * K * B / (ms * 1e-3)
+    if a.dump_outputs:
+        dump_outputs(model, epoch_loss, a.dump_outputs)
 
     # ---- end to end through the public API (host ids) -------------------
     e2e = None

@@ -18,13 +18,14 @@ Contents (every function cites the reference file:line it restates):
 * ``torch_port``-- the reference's fit() loop restated on stock torch CPU ops
                    (the timed ``cpu_baseline`` "port", used by bench.py only when
                    the unmodified reference is not installed under
-                   ``baseline/_ref``).
+                   ``oracle/_ref``).
+* ``reference`` -- installs that unmodified reference under ``oracle/_ref``.
 
 The reference is pure Python (no C sources to compile into ``oracle/_ref``); the
 restatements are NumPy, so there is no C build step for the oracle.
 
 Parity pinning: the restatements are checked (tests/test_oracle_*.py) against
-golden vectors produced by the *live* reference in the build container
-(``tests/golden/make_golden.py`` imports ``/root/reference``), against NumPy's
-own ``RandomState`` and against ``sklearn.utils.murmurhash3_32``.
+golden vectors produced by the *live* reference (``tests/golden/make_golden.py``
+imports a checkout of it), against NumPy's own ``RandomState`` and against
+``sklearn.utils.murmurhash3_32`` (recorded there too).
 """

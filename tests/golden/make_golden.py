@@ -268,9 +268,23 @@ def to_sequence_case():
     np.savez_compressed(os.path.join(HERE, 'to_sequence.npz'), **out)
 
 
+def murmur_case():
+    """sklearn.utils.murmurhash3_32, the hash the reference's BloomEmbedding calls
+    (spotlight/layers.py:7,183), on the int32 edge values, a contiguous span and a seeded
+    sample of the whole int32 range, for the seeds the tests use."""
+    from sklearn.utils import murmurhash3_32
+    rs = np.random.RandomState(11)
+    keys = np.concatenate([np.arange(-5, 1000), [2**31 - 1, -2**31, 2**31 - 2, -2**31 + 1],
+                           rs.randint(-2**31, 2**31 - 1, 4000, dtype=np.int64)]).astype(np.int32)
+    seeds = np.array([0, 179424941, 179426549, 2**32 - 1], dtype=np.uint32)
+    hashes = np.stack([murmurhash3_32(keys, seed=int(s)) for s in seeds]).astype(np.int32)
+    np.savez_compressed(os.path.join(HERE, 'murmur_sklearn.npz'), keys=keys, seeds=seeds, hashes=hashes)
+
+
 if __name__ == '__main__':
     rng_case()
     to_sequence_case()
+    murmur_case()
     for loss in ('pointwise', 'bpr', 'hinge', 'adaptive_hinge'):
         mf_case('mf_' + loss, loss, num_users=97, num_items=53, dim=32, batch=192)
     mf_case('mf_bpr_d64', 'bpr', num_users=300, num_items=41, dim=64, batch=256)

@@ -212,8 +212,8 @@ def test_fused_adam_schedule_and_dense_fallback():
 
 
 def test_reference_arm_prints_the_contract_line():
-    """`bench.py --impl reference` (the arm the driver times beside ours): runs the
-    reference's own fit loop (baseline/_ref when installed, else the oracle port) on the
+    """`bench.py --impl reference` (the CPU arm timed beside ours): runs the
+    reference's own fit loop (oracle/_ref when installed, else the oracle port) on the
     host cores and prints one JSON line with the contract's keys.  Tiny workload here."""
     import json
     import subprocess
@@ -230,7 +230,10 @@ def test_reference_arm_prints_the_contract_line():
     assert line['steps'] == 2 and line['warmup'] == 1 and line['n_gpus'] == 1
     assert line['value'] > 0 and line['higher_is_better'] is True
     cb = line['cpu_baseline']
-    assert cb['kind'] in ('reference', 'port') and cb['cores'] >= 1 and cb['value'] == line['value']
+    # the unmodified reference whenever build() installed it; the torch restatement only without it
+    installed = os.path.isdir(os.path.join(ROOT, 'oracle', '_ref', 'spotlight'))
+    assert cb['kind'] == ('reference' if installed else 'port')
+    assert cb['cores'] >= 1 and cb['value'] == line['value']
     assert line['e2e']['value'] == line['value']
     assert line['e2e']['h2d_bytes_per_step'] == 0 and line['e2e']['d2h_bytes_per_step'] == 0
     assert 'workload' in line['config'] and 'model' not in line['config']

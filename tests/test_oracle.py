@@ -1,5 +1,5 @@
 """Pin the oracle (oracle/*.py) against the live reference's golden vectors,
-NumPy's RandomState and sklearn's murmurhash3_32.  CPU only."""
+NumPy's RandomState and sklearn's murmurhash3_32 (recorded).  CPU only."""
 
 import numpy as np
 import pytest
@@ -65,7 +65,15 @@ def test_jump_table_matches_sequential_twists():
 
 
 def test_murmur_matches_sklearn():
-    sk = pytest.importorskip('sklearn.utils').murmurhash3_32
+    """Against sklearn.utils.murmurhash3_32 (the reference's BloomEmbedding hash) as recorded in
+    tests/golden/murmur_sklearn.npz, and against the live function too where sklearn is installed."""
+    g = load_golden('murmur_sklearn')
+    for s, want in zip(g['seeds'], g['hashes']):
+        assert (murmurhash3_32(g['keys'], int(s)) == want).all(), int(s)
+    try:
+        from sklearn.utils import murmurhash3_32 as sk
+    except ImportError:
+        return
     k = np.concatenate([np.arange(-5, 20000), [2**31 - 1, -2**31]]).astype(np.int32)
     for s in (0, 179424941, 179426549, 2**32 - 1):
         assert (sk(k, seed=s) == murmurhash3_32(k, s)).all()
