@@ -31,7 +31,7 @@ EXPORTS = (
     'slb_embedding_forward', 'slb_bloom_rows',
     'slb_embedding_backward_workspace_bytes', 'slb_embedding_backward',
     'slb_mf_scores', 'slb_mf_scores_backward', 'slb_rank_pairs', 'slb_mf_step_workspace_bytes', 'slb_mf_fused_workspace_bytes', 'slb_mf_compact_rows',
-    'slb_mf_train_step', 'slb_mf_train_step_phases', 'slb_mf_fit_epoch', 'slb_mf_fit_epoch_events', 'slb_adam_flush',
+    'slb_mf_train_step', 'slb_mf_train_step_phases', 'slb_mf_plan_copy', 'slb_mf_fused_layout', 'slb_mf_fit_epoch', 'slb_mf_fit_epoch_events', 'slb_adam_flush',
     'slb_mf_bloom_workspace_bytes', 'slb_mf_bloom_train_step',
     'slb_bias_sparse_workspace_bytes', 'slb_bias_sparse_apply',
     'slb_unique_workspace_bytes', 'slb_unique_bucket', 'slb_shard_gather_batch', 'slb_adagrad_dense',
@@ -140,6 +140,9 @@ def _declare(lib):
     lib.slb_mf_compact_rows.restype = c_i64
     lib.slb_mf_train_step.argtypes = [P(MfStepArgs), c_vp]
     lib.slb_mf_train_step_phases.argtypes = [P(MfStepArgs), c_i32, c_vp]
+    lib.slb_mf_fused_layout.argtypes = [P(MfStepArgs), c_vp, c_i32]
+    lib.slb_mf_fused_layout.restype = c_i32
+    lib.slb_mf_plan_copy.argtypes = [P(MfStepArgs), c_i32, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
     lib.slb_mf_bloom_workspace_bytes.argtypes = [P(MfBloomArgs)]
     lib.slb_mf_bloom_workspace_bytes.restype = c_sz
     lib.slb_mf_bloom_train_step.argtypes = [P(MfBloomArgs), c_vp]

@@ -33,11 +33,18 @@ static inline size_t slb_align_up(size_t x, size_t a) { return (x + a - 1) / a *
 struct WsCarver {
     char* base;
     size_t off;
+    int64_t* log = nullptr;      // optional: [begin, end) byte offsets of every take, up to max_log
+    int n_log = 0, max_log = 0;
     explicit WsCarver(void* p) : base(static_cast<char*>(p)), off(0) {}
     template <typename T>
     T* take(size_t count) {
         off = slb_align_up(off, 256);
         T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+        if (log && n_log < max_log) {
+            log[2 * n_log] = static_cast<int64_t>(off);
+            log[2 * n_log + 1] = static_cast<int64_t>(off + count * sizeof(T));
+        }
+        if (log) ++n_log;
         off += count * sizeof(T);
         return p;
     }

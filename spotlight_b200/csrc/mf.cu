@@ -23,6 +23,8 @@
 //   forward 3R + 3*4 + 3*8, backward re-reads 4R (partner rows), writes <= 3R.
 #include <stdlib.h>
 
+#include <algorithm>
+
 #include "segindex.cuh"
 
 namespace {
@@ -1235,13 +1237,14 @@ struct V2Layout {
     size_t bytes;
 };
 
-V2Layout v2_layout(void* base, int64_t B, int64_t U, int64_t I, int D) {
-    WsCarver ws(base);
+// B is the layout's capacity; a step over fewer interactions passes its own count to the kernels.
+// `log` (optional) receives the [begin, end) byte offsets of every array taken.
+V2Layout v2_layout(void* base, int64_t B, int64_t U, int64_t I, int D, WsCarver* log = nullptr) {
+    WsCarver own(base);
+    WsCarver& ws = log ? *log : own;
     V2Layout l;
     const int64_t R = U + I;
     const int64_t Rpad = (R + SEG_SCAN_TILE - 1) / SEG_SCAN_TILE * SEG_SCAN_TILE;
-    // zero-at-rest state first, at offsets that do not depend on the batch size: one workspace then
-    // serves any batch up to its capacity (the sharded step's local batch changes every step)
     l.st.done = ws.take<int32_t>(8);
     int32_t* cnt[2] = {ws.take<int32_t>(Rpad), ws.take<int32_t>(Rpad)};
     for (int k = 0; k < 2; ++k) {
@@ -1268,6 +1271,9 @@ V2Layout v2_layout(void* base, int64_t B, int64_t U, int64_t I, int D) {
         p.mi_tmp = ws.take<IRec>(2 * B + 1);
         p.words = (2 * B + 31) / 32;
         p.bits = ws.take<uint32_t>(static_cast<size_t>(SEG_LONG_CTAS) * 2 * p.words);
+        p.slot = ws.take<int32_t>(3 * B);
+        p.multi = ws.take<int32_t>(3 * B / 2 + 1);
+        p.nmulti = ws.take<int32_t>(8);
         p.B = B; p.U = U; p.I = I;
         p.err = nullptr; p.users = nullptr; p.items = nullptr; p.negs = nullptr;
     }
@@ -1296,21 +1302,19 @@ int v2_launch_plan(const slb_mf_step_args* x, PlanDev p, int32_t* err, const int
                    const int64_t* negs, int64_t B, cudaStream_t st) {
     p.B = B; p.users = users; p.items = items; p.negs = negs; p.err = err;
     p.seg.long_cap = seg_sort_cap(lpr_for_dim(x->dim));
-    const int sms = slb_sms();
-    int g = static_cast<int>((B + 255) / 256);
-    if (g > sms * 8) g = sms * 8;
+    const int64_t cap = static_cast<int64_t>(slb_sms()) * PLAN_GRID_PER_SM;
+    const int g = static_cast<int>(std::min<int64_t>((B + 255) / 256, cap));
     plan_count_kernel<<<g, 256, 0, st>>>(p);
     SLB_LAUNCH_CHECK("plan_count_kernel");
-    seg_scan_launch(p.seg, p.U, st);
-    SLB_LAUNCH_CHECK("seg_scan_kernel");
+    plan_scan_kernel<<<static_cast<unsigned>(p.seg.ntiles), SEG_SCAN_THREADS, 0, st>>>(p);
+    SLB_LAUNCH_CHECK("plan_scan_kernel");
     plan_fill_kernel<<<g, 256, 0, st>>>(p);
     SLB_LAUNCH_CHECK("plan_fill_kernel");
-    int64_t tiles = ((3 * B + 31) / 32 + 3) / 4;
-    int sg = static_cast<int>(tiles < static_cast<int64_t>(sms) * 16 ? tiles : static_cast<int64_t>(sms) * 16);
-    plan_sort_kernel<<<sg, 128, 0, st>>>(p, p.seg.long_cap);
+    // sort: hot-row blocks first, then enough warps for the longest possible `multi` list, capped
+    const int64_t tiles = ((3 * B / 2 + 1 + 31) / 32 + PLAN_SORT_THREADS / 32 - 1) / (PLAN_SORT_THREADS / 32);
+    const int sg = SEG_LONG_CTAS + static_cast<int>(std::min<int64_t>(tiles, 2 * cap));
+    plan_sort_kernel<<<sg, PLAN_SORT_THREADS, 0, st>>>(p, p.seg.long_cap);
     SLB_LAUNCH_CHECK("plan_sort_kernel");
-    plan_sort_long_kernel<<<SEG_LONG_CTAS, 256, 0, st>>>(p);          // no-op unless hot rows exist
-    SLB_LAUNCH_CHECK("plan_sort_long_kernel");
     return SLB_OK;
 }
 
@@ -1408,6 +1412,27 @@ int v2_check_ws(const slb_mf_step_args* x) {
     return SLB_OK;
 }
 
+// The capacity a fused workspace is laid out for: the largest batch whose layout fits its bytes.
+// It depends on the workspace alone, never on the calling step's batch, so every call sharing a
+// workspace sees the same offsets.  That matters while two steps are in flight with different
+// batches (the sharded step's local batch changes every step, and the plan of step k+1 runs under
+// the float kernels of step k): neither plan slot then lands on the other, or on the step state.
+int64_t v2_capacity(size_t bytes, int64_t U, int64_t I, int D) {
+    int64_t lo = 0, hi = static_cast<int64_t>(bytes / (4 * static_cast<size_t>(D))) + 1;   // the stash alone
+    while (hi - lo > 1) {                                                                 // outgrows `hi`
+        const int64_t mid = lo + (hi - lo) / 2;
+        if (v2_layout(nullptr, mid, U, I, D).bytes <= bytes) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// The layout every call on x->fused_workspace uses (after v2_check_ws: capacity >= x->batch).
+V2Layout v2_layout_ws(const slb_mf_step_args* x, void* base, WsCarver* log = nullptr) {
+    return v2_layout(base, v2_capacity(x->fused_workspace_bytes, x->num_users, x->num_items, x->dim),
+                     x->num_users, x->num_items, x->dim, log);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1434,7 +1459,7 @@ int slb_mf_train_step(const slb_mf_step_args* x, slb_stream_t stream) {
     if (v2_eligible(x)) {
         const int r2 = v2_check_ws(x);
         if (r2 != SLB_OK) return r2;
-        const V2Layout l = v2_layout(x->fused_workspace, x->batch, x->num_users, x->num_items, x->dim);
+        const V2Layout l = v2_layout_ws(x, x->fused_workspace);
         MfLayout old = mf_layout(x->workspace, x->batch, x->num_users, x->num_items);
         return v2_launch_step(x, l, 0, old.err, x->users, x->items, x->negs, x->batch, x->loss_out,
                               static_cast<cudaStream_t>(stream), 7);
@@ -1449,13 +1474,69 @@ int slb_mf_train_step_phases(const slb_mf_step_args* x, int32_t phases, slb_stre
     if (v2_eligible(x)) {          // planned step: 1 plan, 2 user kernels, 4 item kernels
         const int r2 = v2_check_ws(x);
         if (r2 != SLB_OK) return r2;
-        const V2Layout l = v2_layout(x->fused_workspace, x->batch, x->num_users, x->num_items, x->dim);
+        const V2Layout l = v2_layout_ws(x, x->fused_workspace);
         MfLayout old = mf_layout(x->workspace, x->batch, x->num_users, x->num_items);
         return v2_launch_step(x, l, (phases >> 8) & 1, old.err, x->users, x->items, x->negs, x->batch, x->loss_out,
                               static_cast<cudaStream_t>(stream), phases & 7);
     }
     return launch_step(x, x->users, x->items, x->negs, x->batch, x->loss_out,
                        static_cast<cudaStream_t>(stream), phases);
+}
+
+int slb_mf_plan_copy(const slb_mf_step_args* x, int32_t slot, int64_t batch, int32_t* totals, int32_t* seg_row,
+                     int32_t* seg_start, int32_t* sid, int32_t* long_list, void* mu, void* mi, slb_stream_t stream) {
+    SLB_REQUIRE(x && x->fused_workspace && v2_dim_ok(x->dim), "mf_plan_copy: needs a planned-step workspace");
+    SLB_REQUIRE(slot == 0 || slot == 1, "mf_plan_copy: slot must be 0 or 1");
+    SLB_REQUIRE(batch > 0 && batch <= x->batch, "mf_plan_copy: batch must be in [1, args.batch]");
+    SLB_REQUIRE(totals && seg_row && seg_start && sid && long_list && mu && mi, "mf_plan_copy: null output");
+    const int r = v2_check_ws(x);
+    if (r != SLB_OK) return r;
+    const PlanDev& p = v2_layout_ws(x, x->fused_workspace).plan[slot];
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const auto copy = [&](void* dst, const void* src, size_t n) {
+        return cudaMemcpyAsync(dst, src, n, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    };
+    const bool ok = copy(totals, p.seg.totals, 4 * sizeof(int32_t)) &&
+                    copy(seg_row, p.seg.seg_row, (3 * batch + 1) * sizeof(int32_t)) &&
+                    copy(seg_start, p.seg.seg_start, (3 * batch + 2) * sizeof(int32_t)) &&
+                    copy(sid, p.seg.sid, (x->num_users + x->num_items) * sizeof(int32_t)) &&
+                    copy(long_list, p.seg.long_list, (3 * batch / 16 + 2) * sizeof(int32_t)) &&
+                    copy(mu, p.mu, batch * sizeof(URec)) && copy(mi, p.mi, 2 * batch * sizeof(IRec));
+    if (!ok) { slb_set_error("mf_plan_copy: cudaMemcpyAsync failed"); return SLB_ECUDA; }
+    return SLB_OK;
+}
+
+int32_t slb_mf_fused_layout(const slb_mf_step_args* x, int64_t* out, int32_t max_arrays) {
+    SLB_REQUIRE(x && v2_dim_ok(x->dim) && x->batch > 0 && x->num_users > 0 && x->num_items > 0,
+                "mf_fused_layout: needs batch, num_users, num_items and a planned-step dim");
+    SLB_REQUIRE(out || max_arrays == 0, "mf_fused_layout: null output");
+    const int r = v2_check_ws(x);
+    if (r != SLB_OK) return r;
+    // a stand-in base address, never dereferenced: the layout's pointers become byte offsets
+    char* const base = reinterpret_cast<char*>(static_cast<uintptr_t>(1) << 40);
+    int64_t log[2 * 64];
+    WsCarver ws(base);
+    ws.log = log;
+    ws.max_log = 64;
+    const V2Layout l = v2_layout_ws(x, base, &ws);
+    SLB_REQUIRE(ws.n_log <= 64, "mf_fused_layout: more arrays than expected");
+    const auto at = [&](const void* q) { return static_cast<int64_t>(static_cast<const char*>(q) - base); };
+    for (int n = 0; n < ws.n_log && n < max_arrays; ++n) {
+        int64_t group = -1;
+        for (int k = 0; k < 2; ++k) {
+            const PlanDev& p = l.plan[k];
+            const void* mine[] = {p.seg.cnt, p.seg.off, p.seg.sid, p.seg.status, p.seg.ticket, p.seg.seg_row,
+                                  p.seg.seg_start, p.seg.long_list, p.mu, p.mi, p.mu_tmp, p.mi_tmp, p.bits,
+                                  p.slot, p.multi, p.nmulti};
+            for (const void* q : mine) if (at(q) == log[2 * n]) group = k;
+        }
+        const void* step[] = {l.st.done, l.st.t_g, l.st.stash, l.st.partial, l.st.partial_long};
+        for (const void* q : step) if (at(q) == log[2 * n]) group = 2;
+        out[3 * n] = group;
+        out[3 * n + 1] = log[2 * n];
+        out[3 * n + 2] = log[2 * n + 1];
+    }
+    return ws.n_log;
 }
 
 static int fit_epoch_impl(const slb_mf_step_args* x, const int64_t* users, const int64_t* items,
@@ -1474,7 +1555,7 @@ static int fit_epoch_impl(const slb_mf_step_args* x, const int64_t* users, const
         // stream before the float kernels of step k, double-buffered, so it runs under them
         const int r2 = v2_check_ws(&tmp);
         if (r2 != SLB_OK) return r2;
-        const V2Layout l = v2_layout(x->fused_workspace, x->batch, x->num_users, x->num_items, x->dim);
+        const V2Layout l = v2_layout_ws(x, x->fused_workspace);
         MfLayout old = mf_layout(x->workspace, x->batch, x->num_users, x->num_items);
         cudaStream_t plan_st = x->plan_stream ? static_cast<cudaStream_t>(x->plan_stream) : main_st;
         const bool two = plan_st != main_st;

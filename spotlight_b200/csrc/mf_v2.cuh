@@ -37,6 +37,9 @@ struct PlanDev {
     IRec* mi_tmp;          // [2B]
     uint32_t* bits;        // [SEG_LONG_CTAS][2 * words] bitmap + prefix of the hot-row sort
     int64_t words;
+    int32_t* slot;         // [3B]  a member's place in its row's list: the count's atomicAdd (u, i, j blocks)
+    int32_t* multi;        // [3B / 2 + 1] segments with 2..long_cap members, in no particular order
+    int32_t* nmulti;       // [1]   length of `multi`
     int32_t* err;
     int64_t B, U, I;
     const int64_t* users; const int64_t* items; const int64_t* negs;
@@ -51,32 +54,173 @@ struct StepV2 {
 };
 
 // ------------------------------------------------------------------ plan kernels
+//
+// count -> scan -> fill -> sort, four launches.  The plan runs under the previous step's float
+// kernels, so what it costs the step is mostly the SM time its CTAs take from them: the kernels
+// are small grid-stride grids (PLAN_GRID_PER_SM CTAs per SM) with short dependence chains.
 
+#ifndef PLAN_GRID_PER_SM
+#define PLAN_GRID_PER_SM 4
+#endif
+
+__device__ __forceinline__ bool plan_ids_ok(const PlanDev& p, int64_t u, int64_t i, int64_t j) {
+    return u >= 0 && u < p.U && i >= 0 && i < p.I && j >= 0 && j < p.I;
+}
+
+// Counts the members of every row and keeps each member's slot (the value its atomicAdd returned):
+// the fill then places it at off[row] + slot without a second round of atomics.  Also re-arms this
+// plan's scan (look-back words, tile ticket, list lengths); the previous scan of the same plan slot
+// has completed, by stream order.
 __global__ void __launch_bounds__(256) plan_count_kernel(PlanDev p) {
+    const int64_t tid = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     const int64_t nth = static_cast<int64_t>(gridDim.x) * blockDim.x;
-    if (blockIdx.x == 0 && threadIdx.x == 0) p.seg.totals[3] = 0;
-    for (int64_t b = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; b < p.B; b += nth) {
+    for (int64_t t = tid; t < p.seg.ntiles; t += nth) p.seg.status[t] = 0ull;
+    if (tid == 0) { *p.seg.ticket = 0; p.seg.totals[3] = 0; *p.nmulti = 0; }
+    for (int64_t b = tid; b < p.B; b += nth) {
         const int64_t u = p.users[b], i = p.items[b], j = p.negs[b];
-        if (u < 0 || u >= p.U || i < 0 || i >= p.I || j < 0 || j >= p.I) { atomicExch(p.err, 1); continue; }
-        atomicAdd(p.seg.cnt + u, 1);
-        atomicAdd(p.seg.cnt + p.U + i, 1);
-        atomicAdd(p.seg.cnt + p.U + j, 1);
+        if (!plan_ids_ok(p, u, i, j)) { atomicExch(p.err, 1); continue; }
+        const int su = atomicAdd(p.seg.cnt + u, 1);
+        const int si = atomicAdd(p.seg.cnt + p.U + i, 1);
+        const int sj = atomicAdd(p.seg.cnt + p.U + j, 1);
+        p.slot[b] = su;
+        p.slot[p.B + b] = si;
+        p.slot[2 * p.B + b] = sj;
     }
 }
 
+// Single-pass scan of cnt[0..Rpad) (decoupled look-back over dynamically numbered tiles: a tile
+// only waits for tiles that took their number earlier, so it needs no co-residency).  Warp w of a
+// tile owns rows tile * 4096 + w * 512 + 32 k + lane, so every load and store of a warp covers
+// consecutive rows.  Emits off / sid per touched row, the segment list (seg_row, seg_start),
+// long_list (> long_cap members), `multi` (2..long_cap members: the sort's work list) and the
+// totals, and zeroes the counters it consumed.
+constexpr int PLAN_SCAN_WARPS = SEG_SCAN_THREADS / 32;
+constexpr int PLAN_SCAN_ITEMS = SEG_SCAN_TILE / SEG_SCAN_THREADS;     // rows per lane
+
+__global__ void __launch_bounds__(SEG_SCAN_THREADS) plan_scan_kernel(PlanDev p) {
+    __shared__ uint32_t sh_w[3][PLAN_SCAN_WARPS];      // per warp: sum, non-zero rows, multi rows
+    __shared__ uint32_t sh_pre[3];                     // tile prefix: sum, segments, multi position
+    __shared__ int sh_tile;
+    const SegIndex& s = p.seg;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int cap = s.long_cap;
+    if (threadIdx.x == 0) sh_tile = atomicAdd(s.ticket, 1);
+    __syncthreads();
+    const int tile = sh_tile;
+    const int64_t base = static_cast<int64_t>(tile) * SEG_SCAN_TILE + warp * (32 * PLAN_SCAN_ITEMS) + lane;
+
+    int32_t c[PLAN_SCAN_ITEMS];
+#pragma unroll
+    for (int k = 0; k < PLAN_SCAN_ITEMS; ++k) c[k] = s.cnt[base + 32 * k];
+    uint32_t tsum = 0, tnz = 0, tmul = 0;
+#pragma unroll
+    for (int k = 0; k < PLAN_SCAN_ITEMS; ++k) {
+        tsum += c[k]; tnz += c[k] != 0; tmul += c[k] >= 2 && c[k] <= cap;
+        if (c[k] != 0) s.cnt[base + 32 * k] = 0;        // zero at rest again
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        tsum += __shfl_xor_sync(0xffffffffu, tsum, o);
+        tnz += __shfl_xor_sync(0xffffffffu, tnz, o);
+        tmul += __shfl_xor_sync(0xffffffffu, tmul, o);
+    }
+    if (lane == 0) { sh_w[0][warp] = tsum; sh_w[1][warp] = tnz; sh_w[2][warp] = tmul; }
+    __syncthreads();
+    if (warp == 0) {
+        uint32_t v[3];
+#pragma unroll
+        for (int q = 0; q < 3; ++q) v[q] = lane < PLAN_SCAN_WARPS ? sh_w[q][lane] : 0u;
+        uint32_t inc[3] = {v[0], v[1], v[2]};
+#pragma unroll
+        for (int o = 1; o < PLAN_SCAN_WARPS; o <<= 1)
+#pragma unroll
+            for (int q = 0; q < 3; ++q) {
+                const uint32_t t = __shfl_up_sync(0xffffffffu, inc[q], o);
+                if (lane >= o) inc[q] += t;
+            }
+        uint32_t agg[3];
+#pragma unroll
+        for (int q = 0; q < 3; ++q) agg[q] = __shfl_sync(0xffffffffu, inc[q], PLAN_SCAN_WARPS - 1);
+        if (lane < PLAN_SCAN_WARPS)
+#pragma unroll
+            for (int q = 0; q < 3; ++q) sh_w[q][lane] = inc[q] - v[q];      // exclusive, per warp
+        volatile unsigned long long* st = s.status;
+        if (lane == 0) st[tile] = seg_pack(tile == 0 ? SEG_FLAG_INC : SEG_FLAG_AGG, agg[0], agg[1]);
+        unsigned long long pre = 0;                     // [63:32] segments, [31:0] sum of earlier tiles
+        for (int hi = tile - 1; hi >= 0; hi -= 32) {
+            const int j = hi - lane;
+            unsigned long long w = seg_pack(SEG_FLAG_INC, 0u, 0u);
+            if (j >= 0) do { w = st[j]; } while (seg_flag(w) == 0);
+            const unsigned incm = __ballot_sync(0xffffffffu, seg_flag(w) == SEG_FLAG_INC);
+            const int last = incm ? __ffs(incm) - 1 : 31;     // nearest inclusive prefix ends the walk
+            unsigned long long mine = lane <= last ? (static_cast<unsigned long long>(seg_nz(w)) << 32) | seg_sum(w) : 0ull;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, o);
+            pre += mine;
+            if (incm) break;
+        }
+        if (lane == 0) {
+            const uint32_t psum = static_cast<uint32_t>(pre & 0xffffffffull), pnz = static_cast<uint32_t>(pre >> 32);
+            if (tile > 0) st[tile] = seg_pack(SEG_FLAG_INC, psum + agg[0], pnz + agg[1]);
+            sh_pre[0] = psum;
+            sh_pre[1] = pnz;
+            sh_pre[2] = agg[2] ? static_cast<uint32_t>(atomicAdd(p.nmulti, static_cast<int>(agg[2]))) : 0u;
+        }
+    }
+    __syncthreads();
+    uint32_t run = sh_pre[0] + sh_w[0][warp], seg = sh_pre[1] + sh_w[1][warp], mpos = sh_pre[2] + sh_w[2][warp];
+    const unsigned below = (1u << lane) - 1u;
+    const int64_t RA = p.U;
+#pragma unroll
+    for (int k = 0; k < PLAN_SCAN_ITEMS; ++k) {
+        const int64_t row = base + 32 * k;
+        uint32_t inc = c[k];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
+            if (lane >= o) inc += t;
+        }
+        const bool mul = c[k] >= 2 && c[k] <= cap;
+        const unsigned nzm = __ballot_sync(0xffffffffu, c[k] != 0);
+        const unsigned mm = __ballot_sync(0xffffffffu, mul);
+        const uint32_t my_seg = seg + __popc(nzm & below);
+        if (row == RA) s.totals[2] = static_cast<int32_t>(my_seg);
+        if (c[k] != 0) {
+            const uint32_t my_run = run + inc - c[k];
+            s.off[row] = static_cast<int32_t>(my_run);
+            s.sid[row] = static_cast<int32_t>(my_seg);
+            s.seg_row[my_seg] = static_cast<int32_t>(row);
+            s.seg_start[my_seg] = static_cast<int32_t>(my_run);
+            if (cap > 0 && c[k] > cap) s.long_list[atomicAdd(s.totals + 3, 1)] = static_cast<int32_t>(my_seg);
+            if (mul) p.multi[mpos + __popc(mm & below)] = static_cast<int32_t>(my_seg);
+        }
+        run += __shfl_sync(0xffffffffu, inc, 31);
+        seg += __popc(nzm);
+        mpos += __popc(mm);
+    }
+    if (tile == s.ntiles - 1 && threadIdx.x == SEG_SCAN_THREADS - 1) {
+        s.totals[0] = static_cast<int32_t>(seg);
+        s.totals[1] = static_cast<int32_t>(run);
+        s.seg_start[seg] = static_cast<int32_t>(run);
+        if (RA >= s.Rpad) s.totals[2] = static_cast<int32_t>(seg);
+    }
+}
+
+// Places every member at off[row] + slot: independent loads, no atomics.  Members of a row land in
+// the order of the count's atomics; plan_sort_kernel restores ascending term order.
 __global__ void __launch_bounds__(256) plan_fill_kernel(PlanDev p) {
     const int64_t nth = static_cast<int64_t>(gridDim.x) * blockDim.x;
     const int ubase = p.seg.seg_start[p.seg.totals[2]];     // user-side members come first
     for (int64_t b = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; b < p.B; b += nth) {
         const int64_t u = p.users[b], i = p.items[b], j = p.negs[b];
-        if (u < 0 || u >= p.U || i < 0 || i >= p.I || j < 0 || j >= p.I) continue;
-        const int su = p.seg.off[u] + atomicSub(p.seg.cnt + u, 1) - 1;
+        if (!plan_ids_ok(p, u, i, j)) continue;
+        const int su = p.seg.off[u] + p.slot[b];
+        const int useg = p.seg.sid[u];
+        const int si = p.seg.off[p.U + i] + p.slot[p.B + b] - ubase;
+        const int sj = p.seg.off[p.U + j] + p.slot[2 * p.B + b] - ubase;
         URec r;
         r.b = static_cast<int32_t>(b); r.i = static_cast<int32_t>(i); r.j = static_cast<int32_t>(j); r.pad = 0;
         p.mu[su] = r;
-        const int useg = p.seg.sid[u];
-        const int si = p.seg.off[p.U + i] + atomicSub(p.seg.cnt + p.U + i, 1) - 1 - ubase;
-        const int sj = p.seg.off[p.U + j] + atomicSub(p.seg.cnt + p.U + j, 1) - 1 - ubase;
         IRec a; a.t = static_cast<int32_t>(2 * b); a.useg = useg;
         IRec c; c.t = static_cast<int32_t>(2 * b + 1); c.useg = useg;
         p.mi[si] = a;
@@ -106,7 +250,7 @@ __device__ __forceinline__ void rec_set_key(IRec& r, int k) { r.t = k; r.useg = 
 // Sorts each member list of a 32-segment tile ascending by key (the fill placed members in
 // atomic order).  Lists of two: one compare-exchange by the owning lane.  Lists of 3..16: a
 // 16-wide bitonic network over half a warp, one record per lane, two lists per pass.  Lists
-// up to `cap`: ranked by counting by the whole warp.  Hot rows (> cap): plan_sort_long_kernel.
+// up to `cap`: ranked by counting by the whole warp.  Hot rows (> cap): plan_sort_long_one.
 // `len` is 0 for the lanes whose segment belongs to the other table.
 template <typename Rec>
 __device__ __forceinline__ void plan_sort_tile(Rec* base, int start, int len, int cap, Rec* tmp_base) {
@@ -160,30 +304,15 @@ __device__ __forceinline__ void plan_sort_tile(Rec* base, int start, int len, in
     }
 }
 
-__global__ void __launch_bounds__(128) plan_sort_kernel(PlanDev p, int cap) {
-    const int nseg = p.seg.totals[0], nsegA = p.seg.totals[2];
-    const int ubase = p.seg.seg_start[nsegA];
-    const int lane = threadIdx.x & 31;
-    const int ntiles = (nseg + 31) / 32;
-    for (int tile = blockIdx.x * 4 + (threadIdx.x >> 5); tile < ntiles; tile += gridDim.x * 4) {
-        const int s = tile * 32 + lane;
-        int start = 0, len = 0;
-        if (s < nseg) { start = p.seg.seg_start[s]; len = p.seg.seg_start[s + 1] - start; }
-        // a tile may straddle the user / item boundary: two passes with the other half masked
-        plan_sort_tile<URec>(p.mu, start, (s < nsegA) ? len : 0, cap, p.mu_tmp);
-        plan_sort_tile<IRec>(p.mi, start - ubase, (s >= nsegA && s < nseg) ? len : 0, cap, p.mi_tmp);
-    }
-}
-
 // Hot rows: keys are distinct and < nbits, so the rank of a record is the number of set bits
 // below its key in a bitmap of the list (bitmap -> per-word prefix popcount -> rank).
-template <typename Rec>
+template <int NT, typename Rec>
 __device__ void plan_sort_long_one(Rec* base, Rec* tmp, int start, int len, uint32_t* bits, uint32_t* pre,
                                    int W, uint32_t* sh_scan) {
-    const int per = (W + 255) / 256;
-    for (int w = threadIdx.x; w < W; w += 256) bits[w] = 0u;
+    const int per = (W + NT - 1) / NT;
+    for (int w = threadIdx.x; w < W; w += NT) bits[w] = 0u;
     __syncthreads();
-    for (int i = threadIdx.x; i < len; i += 256) {
+    for (int i = threadIdx.x; i < len; i += NT) {
         const int t = rec_key(base[start + i]);
         atomicOr(bits + (t >> 5), 1u << (t & 31));
     }
@@ -193,7 +322,7 @@ __device__ void plan_sort_long_one(Rec* base, Rec* tmp, int start, int len, uint
     for (int w = lo; w < hi; ++w) sum += __popc(bits[w]);
     sh_scan[threadIdx.x] = sum;
     __syncthreads();
-    for (int o = 1; o < 256; o <<= 1) {
+    for (int o = 1; o < NT; o <<= 1) {
         const uint32_t v = threadIdx.x >= o ? sh_scan[threadIdx.x - o] : 0u;
         __syncthreads();
         sh_scan[threadIdx.x] += v;
@@ -202,30 +331,55 @@ __device__ void plan_sort_long_one(Rec* base, Rec* tmp, int start, int len, uint
     uint32_t run = sh_scan[threadIdx.x] - sum;
     for (int w = lo; w < hi; ++w) { pre[w] = run; run += __popc(bits[w]); }
     __syncthreads();
-    for (int i = threadIdx.x; i < len; i += 256) {
+    for (int i = threadIdx.x; i < len; i += NT) {
         const Rec x = base[start + i];
         const int t = rec_key(x);
         const uint32_t r = pre[t >> 5] + __popc(bits[t >> 5] & ((1u << (t & 31)) - 1u));
         tmp[start + r] = x;
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < len; i += 256) base[start + i] = tmp[start + i];
+    for (int i = threadIdx.x; i < len; i += NT) base[start + i] = tmp[start + i];
     __syncthreads();
 }
 
-__global__ void __launch_bounds__(256) plan_sort_long_kernel(PlanDev p) {
-    __shared__ uint32_t sh_scan[256];
-    const int nlong = p.seg.totals[3];
+// The leading SEG_LONG_CTAS blocks sort the hot rows (long_list), one row per block at a time;
+// every other warp takes 32 entries of `multi` at a time.  Rows with one member (three quarters
+// of the user rows of a uniform batch) are never visited.
+constexpr int PLAN_SORT_THREADS = 128;
+
+__global__ void __launch_bounds__(PLAN_SORT_THREADS) plan_sort_kernel(PlanDev p, int cap) {
+    __shared__ uint32_t sh_scan[PLAN_SORT_THREADS];
     const int nsegA = p.seg.totals[2];
     const int ubase = p.seg.seg_start[nsegA];
-    uint32_t* bits = p.bits + static_cast<size_t>(blockIdx.x) * 2 * p.words;
-    uint32_t* pre = bits + p.words;
-    for (int li = blockIdx.x; li < nlong; li += gridDim.x) {
-        const int s = p.seg.long_list[li];
-        const int start = p.seg.seg_start[s];
-        const int len = p.seg.seg_start[s + 1] - start;
-        if (s < nsegA) plan_sort_long_one<URec>(p.mu, p.mu_tmp, start, len, bits, pre, static_cast<int>((p.B + 31) / 32), sh_scan);
-        else plan_sort_long_one<IRec>(p.mi, p.mi_tmp, start - ubase, len, bits, pre, static_cast<int>((2 * p.B + 31) / 32), sh_scan);
+    if (blockIdx.x < SEG_LONG_CTAS) {
+        const int nlong = p.seg.totals[3];
+        uint32_t* bits = p.bits + static_cast<size_t>(blockIdx.x) * 2 * p.words;
+        uint32_t* pre = bits + p.words;
+        for (int li = blockIdx.x; li < nlong; li += SEG_LONG_CTAS) {
+            const int s = p.seg.long_list[li];
+            const int start = p.seg.seg_start[s];
+            const int len = p.seg.seg_start[s + 1] - start;
+            if (s < nsegA)
+                plan_sort_long_one<PLAN_SORT_THREADS, URec>(p.mu, p.mu_tmp, start, len, bits, pre,
+                                                            static_cast<int>((p.B + 31) / 32), sh_scan);
+            else
+                plan_sort_long_one<PLAN_SORT_THREADS, IRec>(p.mi, p.mi_tmp, start - ubase, len, bits, pre,
+                                                            static_cast<int>((2 * p.B + 31) / 32), sh_scan);
+        }
+        return;
+    }
+    constexpr int WARPS = PLAN_SORT_THREADS / 32;
+    const int nmul = *p.nmulti;
+    const int lane = threadIdx.x & 31;
+    const int ntiles = (nmul + 31) / 32;
+    const int wstride = (gridDim.x - SEG_LONG_CTAS) * WARPS;
+    for (int tile = (blockIdx.x - SEG_LONG_CTAS) * WARPS + (threadIdx.x >> 5); tile < ntiles; tile += wstride) {
+        const int k = tile * 32 + lane;
+        int s = -1, start = 0, len = 0;
+        if (k < nmul) { s = p.multi[k]; start = p.seg.seg_start[s]; len = p.seg.seg_start[s + 1] - start; }
+        // a tile mixes user and item segments: two passes with the other side masked
+        plan_sort_tile<URec>(p.mu, start, (s >= 0 && s < nsegA) ? len : 0, cap, p.mu_tmp);
+        plan_sort_tile<IRec>(p.mi, start - ubase, s >= nsegA ? len : 0, cap, p.mi_tmp);
     }
 }
 

@@ -53,10 +53,14 @@ _PLAN_STREAMS = {}
 
 
 def _plan_stream(device):
-    """Per-device stream for the planned step's integer plan kernels (csrc/mf_v2.cuh)."""
+    """Per-device stream for the planned step's integer plan kernels (csrc/mf_v2.cuh).
+
+    Normal priority, like the main stream: the plan has a whole step of float kernels to finish
+    under, and at high priority its blocks are dispatched ahead of theirs and displace them
+    (profiles/plan_overlap.py)."""
     key = torch.device(device).index
     if key not in _PLAN_STREAMS:
-        _PLAN_STREAMS[key] = torch.cuda.Stream(device=device, priority=-1)
+        _PLAN_STREAMS[key] = torch.cuda.Stream(device=device, priority=0)
     return _PLAN_STREAMS[key]
 
 
